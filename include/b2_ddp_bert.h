@@ -326,6 +326,16 @@ int32_t b2_rng_seed(void* rng_state, uint64_t seed, uint64_t step, void* stream)
 int32_t b2_accum_finish(float* src, void* dst, const int64_t* segments /* device [n][3] */, int64_t n_segments,
                         int64_t max_count, void* stream);
 
+/* Gradient accumulation over [begin, end) of the flat space (multiples of 8).
+ * mode 0 (ADD):    acc[e] += scale * float(grads[e])
+ * mode 1 (FINISH): grads[e] = bf16(acc[e] + scale * float(grads[e])); acc[e] = 0
+ * acc fp32, grads bf16 (this micro-batch's gradient, as the backward left it).  128-thread blocks of at most 32
+ * registers and no shared memory: shaped like b2_adamw_background to run per bucket beside the backward's GEMMs. */
+#define B2_ACCUM_ADD 0
+#define B2_ACCUM_FINISH 1
+int32_t b2_grad_accumulate(float* acc, void* grads, int64_t begin, int64_t end, float scale, int32_t mode,
+                           void* stream);
+
 /* bf16 <- fp32 cast of a flat range (initial shadow weights, load_state_dict) and zero fill                 */
 int32_t b2_cast_f32_to_bf16(const float* src, void* dst, int64_t n, void* stream);
 int32_t b2_cast_bf16_to_f32(const void* src, float* dst, int64_t n, void* stream);

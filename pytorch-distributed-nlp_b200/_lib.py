@@ -14,6 +14,7 @@ MAJOR_K, MAJOR_MN = 0, 1
 EPI_NONE, EPI_BIAS, EPI_BIAS_GELU, EPI_BIAS_DROPOUT_RESIDUAL, EPI_RESIDUAL, EPI_GELU_BWD = 0, 1, 2, 3, 4, 5
 EPI_RESIDUAL_F32 = 6
 EPI_ACCUM_F32 = 7
+ACCUM_ADD, ACCUM_FINISH = 0, 1          # b2_grad_accumulate modes
 IPC_HANDLE_BYTES = 64
 FLAG_SLOTS = 64
 
@@ -79,6 +80,7 @@ _SIGNATURES = {
                                C.POINTER(AdamWHParams), vp, vp],
     "b2_adamw_prepare": [C.POINTER(AdamWHParams), vp, vp, vp],
     "b2_adamw_background": [vp, vp, vp, vp, vp, vp, i64, i64, C.POINTER(AdamWHParams), vp, vp],
+    "b2_grad_accumulate": [vp, vp, i64, i64, f32, i32, vp],
     "b2_step_advance": [vp, vp, vp, vp],
     "b2_rng_seed": [vp, u64, u64, vp],
     "b2_cast_f32_to_bf16": [vp, vp, i64, vp],

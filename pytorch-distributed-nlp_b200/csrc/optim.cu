@@ -209,6 +209,48 @@ __global__ void cast_bf16_f32_kernel(const __nv_bfloat16* __restrict__ src, floa
   if (i < n) dst[i] = __bfloat162float(src[i]);
 }
 
+// ---- gradient accumulation (no_sync() micro-batches) ----------------------------------------------------------------
+// Folds one micro-batch's bf16 gradient into the fp32 accumulator: ADD acc += scale * g, FINISH g = bf16(acc + scale *
+// g) and acc = 0.  Launched per bucket under the backward pass (optimizer stream / DDP side stream), so it has the shape
+// of adamw_slim_kernel: 128 threads, at most 32 registers, no shared memory, short-lived blocks; 16-byte accesses
+// (8 elements per thread and iteration).  10 B per parameter for ADD, 12 B for FINISH.
+struct AccumParams {
+  float* acc; __nv_bfloat16* grads;
+  long long begin, nvec8;
+  float scale;
+};
+constexpr int kAccumThreads = 128, kAccumIters = 4;
+template <int MODE>
+__global__ void __launch_bounds__(MODE >= 0 ? kAccumThreads : 0) __maxnreg__(MODE >= 0 ? 32 : 24)
+grad_accumulate_kernel(const AccumParams p) {
+  pdl_wait();
+  pdl_launch_dependents();
+  long long i = (long long)blockIdx.x * (kAccumThreads * kAccumIters) + threadIdx.x;
+#pragma unroll 1
+  for (int it = 0; it < kAccumIters; ++it, i += kAccumThreads) {
+    if (i >= p.nvec8) break;
+    const long long e = p.begin + (i << 3);
+    const uint4 q = *reinterpret_cast<const uint4*>(p.grads + e);
+    float4 a0 = *reinterpret_cast<const float4*>(p.acc + e), a1 = *reinterpret_cast<const float4*>(p.acc + e + 4);
+    a0.x += p.scale * bf16_lo(q.x); a0.y += p.scale * bf16_hi(q.x);
+    a0.z += p.scale * bf16_lo(q.y); a0.w += p.scale * bf16_hi(q.y);
+    a1.x += p.scale * bf16_lo(q.z); a1.y += p.scale * bf16_hi(q.z);
+    a1.z += p.scale * bf16_lo(q.w); a1.w += p.scale * bf16_hi(q.w);
+    if (MODE == B2_ACCUM_ADD) {
+      *reinterpret_cast<float4*>(p.acc + e) = a0;
+      *reinterpret_cast<float4*>(p.acc + e + 4) = a1;
+    } else {
+      uint4 o;
+      o.x = pack_bf16(a0.x, a0.y); o.y = pack_bf16(a0.z, a0.w);
+      o.z = pack_bf16(a1.x, a1.y); o.w = pack_bf16(a1.z, a1.w);
+      *reinterpret_cast<uint4*>(p.grads + e) = o;
+      const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+      *reinterpret_cast<float4*>(p.acc + e) = z;
+      *reinterpret_cast<float4*>(p.acc + e + 4) = z;
+    }
+  }
+}
+
 // segments [n][3] = {src offset, dst offset, count}: dst(bf16) <- src(fp32); src <- 0.  grid = (ceil(max_count/256), n)
 __global__ void accum_finish_kernel(float* __restrict__ src, __nv_bfloat16* __restrict__ dst,
                                     const long long* __restrict__ seg) {
@@ -314,6 +356,36 @@ extern "C" int32_t b2_adamw_background(const void* grads, void* shadow, float* m
   const long long per_block = (long long)kSlimThreads * kSlimIters;
   const long long blocks = (p.nvec4 + per_block - 1) / per_block;
   B2_LAUNCH(adamw_slim_kernel<1>, (unsigned)blocks, kSlimThreads, 0, (cudaStream_t)stream_, p);
+  B2_CUDA(cudaGetLastError());
+  count_launches(1);
+  return 0;
+}
+
+extern "C" int32_t b2_grad_accumulate(float* acc, void* grads, int64_t begin, int64_t end, float scale, int32_t mode,
+                                      void* stream_) {
+  B2_REQUIRE(acc && grads, "grad_accumulate: null pointer");
+  B2_REQUIRE(begin >= 0 && end >= begin && begin % 8 == 0 && end % 8 == 0,
+             "grad_accumulate: range [%lld,%lld) must be 8-element aligned", (long long)begin, (long long)end);
+  B2_REQUIRE(mode == B2_ACCUM_ADD || mode == B2_ACCUM_FINISH, "grad_accumulate: mode %d", mode);
+  if (end == begin) return 0;
+  static bool attr = false;
+  if (!attr) {   // same shared-memory carve-out as the GEMM CTAs it runs beside (see adamw_slim_kernel)
+    B2_CUDA(cudaFuncSetAttribute(grad_accumulate_kernel<B2_ACCUM_ADD>,
+                                 cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    B2_CUDA(cudaFuncSetAttribute(grad_accumulate_kernel<B2_ACCUM_FINISH>,
+                                 cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    attr = true;
+  }
+  AccumParams p;
+  p.acc = acc; p.grads = (__nv_bfloat16*)grads;
+  p.begin = begin; p.nvec8 = (end - begin) >> 3;
+  p.scale = scale;
+  const long long per_block = (long long)kAccumThreads * kAccumIters;
+  const long long blocks = (p.nvec8 + per_block - 1) / per_block;
+  if (mode == B2_ACCUM_ADD)
+    B2_LAUNCH(grad_accumulate_kernel<B2_ACCUM_ADD>, (unsigned)blocks, kAccumThreads, 0, (cudaStream_t)stream_, p);
+  else
+    B2_LAUNCH(grad_accumulate_kernel<B2_ACCUM_FINISH>, (unsigned)blocks, kAccumThreads, 0, (cudaStream_t)stream_, p);
   B2_CUDA(cudaGetLastError());
   count_launches(1);
   return 0;

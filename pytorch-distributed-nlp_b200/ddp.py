@@ -204,6 +204,12 @@ class DistributedDataParallel(nn.Module):
     def forward(self, *args, **kwargs):
         return self.module(*args, **kwargs)
 
+    def no_sync(self):
+        """torch DDP's ``no_sync()``: backwards of forwards run inside the context add to the local fp32 accumulator,
+        with no exchange; the first backward outside it exchanges the window's sum.  ``optimizer.step()`` after only
+        no_sync() backwards raises (the ranks' gradients were never exchanged)."""
+        return self.module.no_sync()
+
     # ---- checkpoint surface ---------------------------------------------------------------------------------------------
     def load_state_dict(self, state_dict, strict=True, assign=False):
         """`model.load_state_dict(torch.load(ckpt))` on the WRAPPED model (multi-gpu-distributed-cls.py:357-363): keys
@@ -260,13 +266,17 @@ class DistributedDataParallel(nn.Module):
             pass
 
     # ---- hooks called by the engine during backward (autograd thread) -----------------------------------------------
-    def _bucket_ready(self, idx, wg_event=None):
+    def _bucket_ready(self, idx, wg_event=None, fold=None):
         """Bucket `idx` holds this rank's final local gradients once the main stream reaches this point and `wg_event`
         (the weight-gradient stream's marker for the layer) has fired.  With an optimizer attached and overlap on,
         start its exchange + update on the side stream right away so it hides behind the rest of backward.  Only the
-        SIDE stream waits for the weight gradients: the main stream's dgrad chain never parks behind them."""
+        SIDE stream waits for the weight gradients: the main stream's dgrad chain never parks behind them.
+        fold: gradient accumulation (engine.fold).  A no_sync() micro-batch is only added to the local accumulator: no
+        barrier, no exchange.  The last one folds the window's sum into the bf16 gradients BEFORE the bucket's barrier,
+        after which the peers read my slice."""
         opt = self.module._optimizer
-        if self.world == 1 or not self.overlap or opt is None or not getattr(opt, "_armed", False):
+        armed = self.world > 1 and self.overlap and opt is not None and getattr(opt, "_armed", False)
+        if fold is None and not armed:
             return
         eng = self.module._engine
         main = torch.cuda.current_stream(eng.dev)
@@ -276,6 +286,11 @@ class DistributedDataParallel(nn.Module):
         if wg_event is not None:
             self._side.wait_event(wg_event)
         s = self._side.cuda_stream
+        if fold is not None:
+            b0, e0, _lbl = self.module._layout.buckets[idx]
+            eng.fold_range(b0, e0, fold[0], fold[1], s)
+            if fold[0] == L.ACCUM_ADD or not armed:
+                return
         self.comm.barrier(_SLOT_BUCKET0 + idx, s)
         self._exchange_update(opt, idx, s)
         if self._pending is None:
@@ -315,15 +330,19 @@ class DistributedDataParallel(nn.Module):
     def _on_backward_done(self):
         pass
 
-    def consensus_probe(self, probe):
+    def consensus_probe(self, probe, window=None):
         """GradScaler inf check under DDP (multi-gpu-distributed-mp-amp-cls.py:166-171): stock DDP all-reduces the
         gradients before the scaler looks at them, so a non-finite value on ONE rank makes EVERY rank skip the step and
         back off its scale.  Here the scaler only sees the 6-float probe on classifier.bias: poison it on every rank
-        when any rank's probe is non-finite (one scalar exchange through peer memory, no host sync)."""
+        when any rank's probe is non-finite (one scalar exchange through peer memory, no host sync).  window: the
+        probe's value summed over the accumulation window (no_sync), checked as well."""
         if self.world == 1:
             return probe
         eng = self.module._engine
-        bad = (~torch.isfinite(probe)).any().to(torch.float32).reshape(1)
+        bad = (~torch.isfinite(probe)).any()
+        if window is not None:
+            bad = bad | (~torch.isfinite(window)).any()
+        bad = bad.to(torch.float32).reshape(1)
         dst = torch.empty(1, dtype=torch.float32, device=eng.dev)
         L.call("b2_scalar_allreduce_mean", bad.data_ptr(), dst.data_ptr(), L.ptr_array(self.comm.peers["scalar_inf"]),
                L.ptr_array(self.comm.peers["flags"]), self.world, self.rank, _SLOT_INF,

@@ -11,6 +11,7 @@ The arithmetic follows HF ``BertForSequenceClassification`` (SP/transformers/mod
 1077-1154, eager attention) in bf16 with fp32 accumulation/statistics; fp32 master weights stay the parameters
 the user sees.  There is no PyTorch fallback: without the CUDA library every call raises.
 """
+import contextlib
 import os
 from collections import OrderedDict
 
@@ -191,6 +192,7 @@ class _StepFn(torch.autograd.Function):
         logits, loss = eng.forward(input_ids, token_type_ids, attention_mask, labels, training=model.training,
                                    need_backward=True, packed=packed)
         ctx.model = model
+        ctx.no_sync = model._no_sync     # as in torch DDP, whether this micro-batch accumulates is fixed at forward time
         ctx.has_loss = loss is not None
         ctx.set_materialize_grads(False)
         if loss is None:
@@ -204,13 +206,27 @@ class _StepFn(torch.autograd.Function):
         if d_logits is None and (d_loss is None or not ctx.has_loss):
             raise RuntimeError("backward reached the model without any gradient")
         if model._optimizer is not None:
-            # gradients are OVERWRITTEN by every backward (bf16 bucket space, zero_grad is a no-op): a second backward
-            # before optimizer.step() would silently drop the first one's gradients where torch would accumulate
+            # gradients are OVERWRITTEN by every backward outside no_sync() (bf16 bucket space): a second one before
+            # optimizer.step() would silently drop the first one's gradients where torch would accumulate
             if model._grads_live:
                 raise RuntimeError("backward() called twice without optimizer.step() in between: gradient "
-                                   "accumulation is not supported on this path (gradients are overwritten, not summed)")
-            model._grads_live = True
-        eng.backward(d_logits, d_loss if ctx.has_loss else None)
+                                   "accumulation is not supported on this path outside no_sync() (gradients are "
+                                   "overwritten, not summed)")
+            if not ctx.no_sync:
+                model._grads_live = True
+        # no_sync(): this micro-batch is added to the fp32 accumulator.  The first backward outside it folds the
+        # accumulated sum back into the bf16 gradient space, where the exchange and the optimizer read it.
+        if ctx.no_sync:
+            eng.ensure_accum()
+            fold = (L.ACCUM_ADD, 1.0)
+        else:
+            fold = (L.ACCUM_FINISH, 1.0) if eng.accum_pending else None
+        eng.fold = fold
+        try:
+            eng.backward(d_logits, d_loss if ctx.has_loss else None)
+        finally:
+            eng.fold = None
+        eng.accum_pending = eng.accum_pending + 1 if ctx.no_sync else 0
         model._notify_backward_done()
         # Gradients live in the engine's bf16 bucket space, not in `.grad`.  The anchor (classifier.bias) gets its
         # true gradient as a 6-float fp32 probe: it is the column sum of d_logits, so an inf/nan anywhere upstream
@@ -220,8 +236,15 @@ class _StepFn(torch.autograd.Function):
         for d in shape:
             n *= d
         probe = eng.grads[off:off + n].float().view(shape)
-        if model._ddp is not None:
-            probe = model._ddp.consensus_probe(probe)
+        window = probe
+        if fold is not None and fold[0] == L.ACCUM_FINISH:
+            # the gradient space now holds the window's sum; autograd adds the probe to the .grad the earlier
+            # micro-batches left, so return the difference: .grad ends as the window's sum, as torch's would
+            prev = model._params_by_name["classifier.bias"].grad
+            if prev is not None:
+                probe = window - prev
+        if model._ddp is not None and not ctx.no_sync:
+            probe = model._ddp.consensus_probe(probe, window)   # covers every micro-batch of the window
         return probe, None, None, None, None, None, None
 
 
@@ -246,6 +269,7 @@ class BertForSequenceClassification(nn.Module):
         self._optimizer = None
         self._ddp = None
         self._grads_live = False     # an eager backward has produced gradients no optimizer.step() has consumed yet
+        self._no_sync = False        # inside no_sync(): training forwards accumulate their gradients
 
     # ---- module skeleton reproducing HF parameter paths -------------------------------------------------------
     def _build_skeleton(self):
@@ -411,6 +435,19 @@ class BertForSequenceClassification(nn.Module):
                                             training=self.training, need_backward=False, packed=packed)
         return SequenceClassifierOutput(loss=None if loss is None else loss.clone(), logits=logits.clone())
 
+    @contextlib.contextmanager
+    def no_sync(self):
+        """Gradient accumulation, as torch DDP's ``no_sync()``: the backward of a training forward run inside the
+        context ADDS its gradient to the model's fp32 accumulator (no exchange, no update).  The first backward outside
+        it is the window's last micro-batch: the gradient space then holds the sum, and ``optimizer.step()`` applies it.
+        Loss scaling stays with the caller (``criterion(...) / k``).  Needed on one GPU, where there is no wrapper."""
+        prev = self._no_sync
+        self._no_sync = True
+        try:
+            yield
+        finally:
+            self._no_sync = prev
+
     def _notify_backward_done(self):
         if self._ddp is not None:
             self._ddp._on_backward_done()
@@ -453,6 +490,11 @@ class _Engine:
         # backward's fp32 owner-row accumulators ([tokens + seq*types][H] fp32 = 13.4 MB at config A)
         self._ws = {}
         self._saved = None
+        # gradient accumulation (no_sync): fp32 sum over the pending micro-batches of a window, allocated by the first
+        # accumulating backward; `fold` = (b2_grad_accumulate mode, scale) for the backward about to run, or None
+        self.accum = None
+        self.accum_pending = 0
+        self.fold = None
         self.wgrad_stream = torch.cuda.Stream(device=self.dev)
         self.opt_stream = torch.cuda.Stream(device=self.dev)
         self.accum_dgrad = os.environ.get("B2_ACCUM_DGRAD", "1") != "0"
@@ -513,6 +555,22 @@ class _Engine:
 
     def refresh_shadow(self):
         L.call("b2_cast_f32_to_bf16", L.ptr(self.model._flat), L.ptr(self.shadow), self.lay.total, self.stream())
+
+    def ensure_accum(self):
+        """the fp32 accumulator (zeroed; a local buffer, never shared with peers)"""
+        if self.accum is None:
+            self.accum = torch.zeros(self.lay.total, dtype=torch.float32, device=self.dev)
+        return self.accum
+
+    def fold_range(self, begin, end, mode, scale, stream):
+        L.call("b2_grad_accumulate", self.ensure_accum().data_ptr(), self.grads.data_ptr(), begin, end, float(scale),
+               mode, stream)
+
+    def discard_accum(self):
+        """drops the micro-batches not applied yet (optimizer.zero_grad)"""
+        if self.accum_pending:
+            L.call("b2_zero", self.accum.data_ptr(), 4 * self.accum.numel(), self.stream())
+            self.accum_pending = 0
 
     def seed_dropout(self, seed, step=0):
         L.call("b2_rng_seed", L.ptr(self.rng), int(seed), int(step), self.stream())
@@ -806,30 +864,40 @@ class _Engine:
 
         # (head bucket is announced right after these helpers are defined)
         opt = self.model._optimizer
+        fold = self.fold
+        accumulating = fold is not None and fold[0] == L.ACCUM_ADD
         overlap_opt = hooks is None and opt is not None and getattr(opt, "_armed", False)
         # single GPU, optimizer armed by the fused step, no GradScaler: the encoder weight matrices are updated in the
         # epilogue of the grouped weight-gradient GEMM itself (no gradient round trip, no separate HBM-bound pass over
-        # 85 % of the parameters); the per-bucket AdamW launches then skip those vectors
-        self.fused_adamw_active = bool(overlap_opt and self.grouped_wgrad and self.fused_adamw and
+        # 85 % of the parameters); the per-bucket AdamW launches then skip those vectors.  Not while accumulating: that
+        # update would read this micro-batch's gradient instead of the window's sum.
+        self.fused_adamw_active = bool(overlap_opt and self.grouped_wgrad and self.fused_adamw and fold is None and
                                        getattr(opt, "grad_scale", None) is None and
                                        not getattr(opt, "_amp_seen", False))
+        # a world > 1 wrapper folds each bucket on its side stream, ahead of the bucket's barrier (ddp._bucket_ready)
+        ddp_hooks = hooks is not None and hooks.world > 1
+        fold_stream = hooks._side if ddp_hooks else self.opt_stream
 
         def bucket_ready(idx, wg_event=None):
             """bucket `idx` holds its final gradients once the main stream reaches this point (and `wg_event`,
             the weight-gradient stream's marker for the layer, has fired)"""
-            if hooks is not None:
-                hooks._bucket_ready(idx, wg_event)
-            elif overlap_opt:
-                # single GPU: the HBM-bound AdamW of this bucket runs on its own stream under the rest of backward
+            if hooks is not None and (ddp_hooks or fold is None):
+                hooks._bucket_ready(idx, wg_event, fold)
+            elif overlap_opt or fold is not None:
+                # single GPU: the fold and the HBM-bound AdamW of this bucket run on their own stream under the rest
+                # of backward; a non-final micro-batch is only folded
                 ev = torch.cuda.Event()
                 ev.record(main)
                 self.opt_stream.wait_event(ev)
                 if wg_event is not None:
                     self.opt_stream.wait_event(wg_event)
                 b0, e0, _lbl = self.lay.buckets[idx]
-                opt.update_range(b0, e0, 1, 0, [self.grads.data_ptr()], [self.shadow.data_ptr()],
-                                 self.opt_stream.cuda_stream, background=(idx != 0))
-                opt._pending.add(idx)
+                if fold is not None:
+                    self.fold_range(b0, e0, fold[0], fold[1], self.opt_stream.cuda_stream)
+                if overlap_opt and not accumulating:
+                    opt.update_range(b0, e0, 1, 0, [self.grads.data_ptr()], [self.shadow.data_ptr()],
+                                     self.opt_stream.cuda_stream, background=(idx != 0))
+                    opt._pending.add(idx)
 
         if not self.lay.head_in_last_layer:
             bucket_ready(len(self.lay.buckets) - 1)     # (a model without encoder layers: the head is its own bucket)
@@ -943,8 +1011,15 @@ class _Engine:
         # stream's work.  Under an armed DDP exchange the side stream has taken those dependencies bucket by bucket
         # (ddp._bucket_ready) and optimizer.step() joins the side stream; in every other case join here.
         ddp_overlap = (hooks is not None and hooks.world > 1 and hooks.overlap and opt is not None and
-                       getattr(opt, "_armed", False))
+                       getattr(opt, "_armed", False) and not accumulating)
         if side is not main and not ddp_overlap:
             for l in sorted(done)[:2]:       # the last two layers processed (0 and 1) may still be in flight
                 main.wait_event(done[l])
         bucket_ready(0)
+        if fold is not None:
+            # ordering rule of accumulation: the next backward writes gradients (the embedding bucket's clear, the head
+            # gradients) at its very start, so nothing may run on the main stream before every fold has read them
+            main.wait_stream(fold_stream)
+            if accumulating:
+                # one dropout RNG step per micro-batch: micro-batch j of a window draws the masks of step r0 + j
+                L.call("b2_step_advance", None, rng, None, s)

@@ -231,8 +231,11 @@ class AdamW(torch.optim.Optimizer):
     def zero_grad(self, set_to_none=True):
         """Gradients live in the bf16 bucket space and are overwritten by every backward: nothing to clear
         (the reference's zero_grad [:172] exists only because torch accumulates into .grad).  The one real `.grad`
-        is the small fp32 probe the eager backward leaves on classifier.bias for GradScaler's inf check."""
+        is the small fp32 probe the eager backward leaves on classifier.bias for GradScaler's inf check.  Micro-batches
+        accumulated under no_sync() and not applied yet are discarded, as torch discards their .grad."""
         self._model._params_by_name["classifier.bias"].grad = None
+        if self._model._engine is not None:
+            self._model._engine.discard_accum()
         return None
 
     def update_range(self, begin, end, world, rank, peer_grads, peer_shadow, stream, background=False):
@@ -271,10 +274,19 @@ class AdamW(torch.optim.Optimizer):
         if eng is None:
             raise RuntimeError("optimizer.step(): the model is not on CUDA")
         if model._ddp is not None and model._ddp.world > 1:
+            if eng.accum_pending:
+                raise RuntimeError("optimizer.step() after only no_sync() backwards: the last micro-batch of a window "
+                                   "must run outside no_sync(), or the ranks would step on gradients never exchanged")
             model._ddp._optimizer_step(self)
         else:
             main = torch.cuda.current_stream(eng.dev)
             s = main.cuda_stream
+            if eng.accum_pending:
+                # only no_sync() backwards since the last step: apply their sum (the gradient space holds the last
+                # micro-batch, already added, hence scale 0)
+                main.wait_stream(eng.opt_stream)
+                eng.fold_range(0, model._layout.total, L.ACCUM_FINISH, 0.0, s)
+                eng.accum_pending = 0
             if self._pending:
                 ev = torch.cuda.Event()
                 ev.record(eng.opt_stream)

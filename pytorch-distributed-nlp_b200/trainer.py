@@ -9,12 +9,14 @@ Same methods, same argument meaning: ``on_step`` [:126-137], ``loss_reduce`` [:1
   * ``loss_reduce`` / ``output_reduce`` go through the peer-memory kernels when the model is the b200 DDP wrapper;
   * ``train`` uses :class:`FusedTrainStep` (the whole step captured in one CUDA graph) when ``args.fused`` is set.
 """
+import contextlib
 import os
 import time
 
 import numpy as np
 import torch
 
+from . import _lib as L
 from .ddp import DistributedDataParallel
 
 
@@ -40,10 +42,20 @@ class Args:
                           # reference pads every row to max_seq_len although real rows average 18 tokens [:76]
     log_every = 1         # the reference prints every step (forces a D2H sync per step)
     total_step = 0
+    use_grad_accumulation = False   # fabric/fabric-cls.py's accumulation: the loss is divided by grad_accumulation and
+    grad_accumulation = 4           # the optimizer steps when (step + 1) % grad_accumulation == 0 (per-epoch index)
 
 
 def _unwrap(model):
     return model.module if isinstance(model, DistributedDataParallel) else model
+
+
+def _arm_pipelining(optimizer, grad_accumulation):
+    """the pipelined update (optim.AdamW.enable_pipelining) runs on step-local gradients: not while accumulating"""
+    if grad_accumulation == 1:
+        optimizer.enable_pipelining()     # one GPU: the update moves under the NEXT step's forward (optim.py)
+    elif optimizer._pipelined:
+        raise ValueError("gradient accumulation needs the unpipelined update (B2_PIPELINED_ADAMW=0)")
 
 
 class _StagedGraphStep:
@@ -68,6 +80,12 @@ class _StagedGraphStep:
         self.use_graph = use_graph
         self.graph = None
         self._warm = 0
+        # gradient accumulation (train steps built with grad_accumulation > 1): a second graph for the non-final
+        # micro-batches of a window; `_final` selects which one the next run_device() replays
+        self.grad_accumulation = 1
+        self._final = True
+        self._graph_accum = None
+        self._warm_accum = 0
         self._h2d_done = None
         # The step body -- the critical chain of forward / dgrad kernels -- is issued (and captured) on a HIGH-priority
         # stream, so that when an SM frees up the block scheduler hands it to the critical path before the
@@ -117,31 +135,44 @@ class _StagedGraphStep:
             self._body()
         cur.wait_stream(self._prio_stream)
 
-    def run_device(self):
-        """The step with inputs already staged on the device (bench `value` path)."""
+    def run_device(self, final=True):
+        """The step with inputs already staged on the device (bench `value` path).  final=False (train steps built
+        with grad_accumulation > 1): a non-final micro-batch, only added to the accumulator."""
+        k = self.grad_accumulation
+        if not final and k == 1:
+            raise ValueError("a non-final micro-batch needs a train step built with grad_accumulation > 1")
+        self._final = final
+        if k > 1:
+            self.eng.ensure_accum()          # allocated (and zeroed) outside any capture
         self._run_device()
         opt = getattr(self, "opt", None)
         if opt is not None and opt._pipelined:
             opt._deferred_pending = True      # (a graph replay runs no Python: keep the host-side flag current)
+        if k > 1:
+            self.eng.accum_pending = 0 if final else self.eng.accum_pending + 1
 
     def _run_device(self):
         if not self.use_graph:
             self._run_body()
             return
-        if self.graph is None:
-            if self._warm < 2:
+        if not self._final:
+            self._graph_accum, self._warm_accum = self._replay(self._graph_accum, self._warm_accum)
+            return
+        self.graph, self._warm = self._replay(self.graph, self._warm)
+
+    def _replay(self, graph, warm):
+        """one run of the body through `graph`, capturing it after two eager warm-up runs; returns (graph, warm)"""
+        if graph is None:
+            if warm < 2:
                 # eager warm-up: first launches set kernel attributes, DDP arms its overlap path
                 self._run_body()
-                self._warm += 1
-                return
+                return None, warm + 1
             torch.cuda.synchronize(self.eng.dev)
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
                 self._run_body()
-            self.graph = g
-            self.graph.replay()
-            return
-        self.graph.replay()
+        graph.replay()
+        return graph, warm
 
     def _train_body(self, forward):
         """forward(weight_events) -> (logits, loss): the common part of the captured train steps"""
@@ -152,8 +183,20 @@ class _StagedGraphStep:
         eng._saved = None
         Bo = B if packed is None else packed[1].numel()
         ws = eng.workspace(B, S, Bo)
-        # d(loss)/d(logits) was produced by the CE kernel: the reference's criterion(logits, label) [:169]
-        eng._backward_from_dlogits(ws["dloss_logits"], B, S, mask, p_h, p_a, p_c, packed)
+        k = self.grad_accumulation
+        if k > 1:
+            # the reference's loss / k, applied by the fold: ADD for a non-final micro-batch (no update, no exchange),
+            # FINISH ahead of each bucket's update or exchange for the last one
+            eng.fold = (L.ACCUM_FINISH if self._final else L.ACCUM_ADD, 1.0 / k)
+        try:
+            # d(loss)/d(logits) was produced by the CE kernel: the reference's criterion(logits, label) [:169]
+            eng._backward_from_dlogits(ws["dloss_logits"], B, S, mask, p_h, p_a, p_c, packed)
+        finally:
+            eng.fold = None
+        if not self._final:
+            self.loss_out.copy_(loss)
+            return
+        eng.accum_pending = 0
         if opt._pipelined:
             opt.mark_grads_pending()
             torch.cuda.current_stream(eng.dev).wait_stream(eng.opt_stream)   # (step counter bump of the applied update)
@@ -172,13 +215,16 @@ class FusedTrainStep(_StagedGraphStep):
     backward, the peer-HBM gradient exchange fused with AdamW, and the device-side step/RNG bump.  Semantically the body
     of the reference loop [:166-176] without the host round trips."""
 
-    def __init__(self, model, optimizer, batch_size, seq_len, use_graph=True):
+    def __init__(self, model, optimizer, batch_size, seq_len, use_graph=True, grad_accumulation=1):
+        """grad_accumulation = k > 1: micro-batches of a window scaled by 1 / k (the reference's loss / k), the
+        update applied by the call with final=True"""
         super().__init__(model, batch_size, seq_len, use_graph)
         self.opt = optimizer
+        self.grad_accumulation = int(grad_accumulation)
         # the fused step owns backward + optimizer: per-bucket AdamW (and, under DDP, the peer exchange) may start
         # while backward is still running
         optimizer._armed = True
-        optimizer.enable_pipelining()     # one GPU: the update moves under the NEXT step's forward (optim.py)
+        _arm_pipelining(optimizer, self.grad_accumulation)
         self.kernel_launches = None
 
     # the step body, expressed only with stream-ordered work (capturable)
@@ -187,11 +233,11 @@ class FusedTrainStep(_StagedGraphStep):
         self._train_body(lambda ev: self.eng.forward(self.d_ids, self.d_tt, self.d_mask, self.d_lab, training=True,
                                                      need_backward=True, weight_events=ev))
 
-    def __call__(self, batch_data):
+    def __call__(self, batch_data, final=True):
         """batch_data: the dict the reference Collate yields (host int64 tensors).  Returns the device loss scalar
-        (local rank's mean CE, like `loss` at [:169])."""
+        (local rank's mean CE, like `loss` at [:169]).  final=False: a non-final micro-batch (see grad_accumulation)."""
         self.stage(batch_data)
-        self.run_device()
+        self.run_device(final)
         return self.loss_out
 
 
@@ -200,10 +246,11 @@ class PackedTrainStep(_StagedGraphStep):
     instance (staging buffers + CUDA graph) per bin count; the Trainer keeps a small cache of them, since the number of
     bins a batch packs into varies with its lengths."""
 
-    def __init__(self, model, optimizer, bins, batch, use_graph=True):
+    def __init__(self, model, optimizer, bins, batch, use_graph=True, grad_accumulation=1):
         super().__init__(model, bins, 128, use_graph)
         dev = self.eng.dev
         self.bins, self.batch = bins, batch
+        self.grad_accumulation = int(grad_accumulation)
         n = bins * 128
         # pinned staging: ids | token types | positions | segments (as int64) | cls rows | labels
         self.h_stage = torch.empty(4 * n + 2 * batch, dtype=torch.int64).pin_memory()
@@ -213,7 +260,7 @@ class PackedTrainStep(_StagedGraphStep):
         self.d_seg = torch.zeros(bins, 128, dtype=torch.int32, device=dev)
         self.opt = optimizer
         optimizer._armed = True
-        optimizer.enable_pipelining()
+        _arm_pipelining(optimizer, self.grad_accumulation)
 
     def _unstage(self):
         n, st = self.bins * 128, self.d_stage
@@ -246,9 +293,9 @@ class PackedTrainStep(_StagedGraphStep):
         self._train_body(lambda ev: self.eng.forward(self.d_ids, self.d_tt, None, self.d_lab, training=True,
                                                      need_backward=True, packed=packed, weight_events=ev))
 
-    def __call__(self, packed, label):
+    def __call__(self, packed, label, final=True):
         self.stage(packed, label)
-        self.run_device()
+        self.run_device(final)
         return self.loss_out
 
 
@@ -340,36 +387,63 @@ class Trainer:
             return self.model.all_gather_rows(outputs), self.model.all_gather_rows(targets)
         return outputs.clone(), targets.clone()
 
-    def train_step(self, batch_data):
-        """One step of the reference loop body [:166-176]; returns the rank-averaged loss (device scalar)."""
+    def grad_accumulation(self):
+        """micro-batches per optimizer step: args.grad_accumulation under args.use_grad_accumulation, else 1"""
+        if not getattr(self.args, "use_grad_accumulation", False):
+            return 1
+        k = int(getattr(self.args, "grad_accumulation", 1))
+        if k < 1:
+            raise ValueError("grad_accumulation must be >= 1 (got %d)" % k)
+        return k
+
+    def train_step(self, batch_data, step_optimizer=True):
+        """One step of the reference loop body [:166-176]; returns the rank-averaged loss (device scalar).
+        step_optimizer=False: a non-final micro-batch of an accumulation window (fabric/fabric-cls.py:150-161): its
+        loss / k gradient is added to the model's accumulator, with no exchange and no update.  The returned loss is
+        the micro-batch's own, not divided by k."""
+        k = self.grad_accumulation()
+        final = bool(step_optimizer)
         if getattr(self.args, "fused", True) and getattr(self.args, "pack", False) and \
                 batch_data["input_ids"].shape[1] == 128 and not batch_data["input_ids"].is_cuda:
             from .packing import pack_batch
             packed = pack_batch(batch_data["input_ids"], batch_data["token_type_ids"], batch_data["attention_mask"])
             key = (packed["bins"], batch_data["input_ids"].shape[0])
+            if key in self._packed and self._packed[key].grad_accumulation != k:
+                del self._packed[key]
             if key not in self._packed:
                 if len(self._packed) >= 16:           # bound the graph cache: drop the oldest entry
                     self._packed.pop(next(iter(self._packed)))
-                self._packed[key] = PackedTrainStep(self.model, self.optimizer, key[0], key[1])
+                self._packed[key] = PackedTrainStep(self.model, self.optimizer, key[0], key[1], grad_accumulation=k)
             self.model.train()
-            loss = self._packed[key](packed, batch_data["label"])
+            loss = self._packed[key](packed, batch_data["label"], final)
         elif getattr(self.args, "fused", True):
             B, S = batch_data["input_ids"].shape
-            if self._fused is None or (self._fused.B, self._fused.S) != (B, S):
-                self._fused = FusedTrainStep(self.model, self.optimizer, B, S)
+            if self._fused is None or (self._fused.B, self._fused.S, self._fused.grad_accumulation) != (B, S, k):
+                self._fused = FusedTrainStep(self.model, self.optimizer, B, S, grad_accumulation=k)
             self.model.train()
-            loss = self._fused(batch_data)
+            loss = self._fused(batch_data, final)
         elif getattr(self.args, "use_amp", False):
             # the -amp scripts' loop body (multi-gpu-distributed-mp-amp-cls.py:166-171), scaler created once
             if self._scaler is None:
                 self._scaler = torch.amp.GradScaler("cuda")
             self.model.train()
-            with torch.autocast("cuda"):
+            with torch.autocast("cuda"), self._window(final):
                 logits, label = self.on_step(batch_data)
                 loss = self.criterion(logits, label)
-            self._scaler.scale(loss).backward()
-            self._scaler.step(self.optimizer)
-            self._scaler.update()
+            self._scaler.scale(loss / k if k > 1 else loss).backward()
+            if final:
+                self._scaler.step(self.optimizer)
+                self._scaler.update()
+        elif k > 1 or not final:
+            # fabric-cls.py:150-161: loss / k, step and zero_grad once per window
+            self.model.train()
+            with self._window(final):
+                logits, label = self.on_step(batch_data)
+                loss = self.criterion(logits, label)
+            (loss / k).backward()
+            if final:
+                self.optimizer.step()
+                self.optimizer.zero_grad()
         else:
             self.model.train()
             logits, label = self.on_step(batch_data)
@@ -378,6 +452,10 @@ class Trainer:
             loss.backward()
             self.optimizer.step()
         return self.loss_reduce(loss.detach())
+
+    def _window(self, final):
+        """the forward of a non-final micro-batch runs under no_sync()"""
+        return contextlib.nullcontext() if final else self.model.no_sync()
 
     def train(self, train_loader, dev_loader=None, train_sampler=None):
         gloabl_step = 1
@@ -388,7 +466,12 @@ class Trainer:
             if train_sampler is not None:
                 train_sampler.set_epoch(epoch)
             for step, batch_data in enumerate(train_loader):
-                loss = self.train_step(batch_data)
+                if getattr(self.args, "use_grad_accumulation", False):
+                    # per-epoch index, as fabric-cls.py:157: a window left open at the end of an epoch is completed
+                    # by the first micro-batches of the next one
+                    loss = self.train_step(batch_data, step_optimizer=(step + 1) % self.grad_accumulation() == 0)
+                else:
+                    loss = self.train_step(batch_data)
                 if self.args.local_rank == 0 and gloabl_step % max(1, getattr(self.args, "log_every", 1)) == 0:
                     print("【train】 epoch：{}/{} step：{}/{} loss：{:.6f}".format(
                         epoch, self.args.epochs, gloabl_step, self.args.total_step, float(loss)
